@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric: 3-stage 256x256 speech-conditioned StackGAN-v2 TRAIN images/sec.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 24]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 24] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   (N > 1)
 
 One "step" = the reference's inner train loop over one batch (trainer.py:537-572 minus Inception): G forward,
@@ -42,9 +42,12 @@ def workload_name(branches, batch):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (with --sustain: at least this many)")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--impl", default="ours", choices=["ours", "reference"],
+                    help="reference: the train step on the host CPU, the unmodified reference when a checkout of it is "
+                         "given with $SG2_REF or placed at baseline/_ref (kind 'reference'), else the oracle port "
+                         "(kind 'port'); its steps take seconds each, so raise SG2_BENCH_WATCHDOG for long runs")
     ap.add_argument("--batch", type=int, default=24, help="per-GPU batch (birds_3stages.yml: 24)")
     ap.add_argument("--branches", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -57,7 +60,15 @@ def parse():
                     help="keep replaying the step for at least this many seconds before / as the timed region (clocks and "
                          "power settle to the sustained state MEASURED_PEAKS.json's sustained figures refer to)")
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"], help="fp32: the fp32-accurate mode")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0; "
+                         "train: losses and the updated weights, EMA weights and BatchNorm buffers; synth: the images), "
+                         "each array larger than 2^20 elements as a fixed, seeded sample of 2^20 of its elements; "
+                         "not with --sustain, whose step count depends on a measured step time")
+    args = ap.parse_args()
+    if args.dump_outputs and args.sustain > 0:
+        ap.error("--dump-outputs needs a fixed number of steps: leave out --sustain")
+    return args
 
 
 def load_peaks(sustained):
@@ -136,7 +147,7 @@ class ClockSampler:
 def cpu_step_times(batch, branches, steps, warmup, threads):
     """The reference's CPU implementation of the train step on the host cores, fp32 PyTorch/oneDNN: the UNMODIFIED
     reference (condGANTrainer.train_Dnet / train_Gnet on its own G_NET / D_NET*) when a reference tree is available
-    ($SG2_REF, baseline/_ref, /root/reference: oracle/ref_loader.py), else the oracle port of the same algorithm.
+    ($SG2_REF or baseline/_ref: oracle/ref_loader.py), else the oracle port of the same algorithm.
     -> (per-step seconds, kind)"""
     from oracle import ref_loader
     from oracle.stackgan_oracle import Cfg, OracleTrainer, synthetic_batch
@@ -167,18 +178,12 @@ def run_reference(args):
                           "synthesis has no CPU reference leg"}))
         return
     cores = os.cpu_count() or 1
-    # bounded sample of the SAME workload (same batch): the number of steps shrinks, never the batch
-    (probe,), kind = cpu_step_times(args.batch, args.branches, 1, 0, cores)
-    budget = 170.0
     steps, warmup = args.steps, args.warmup
-    if probe * (steps + warmup) > budget:
-        warmup = 1
-        steps = max(3, int(budget / probe) - 2)
     times, kind = cpu_step_times(args.batch, args.branches, steps, warmup, cores)
     ms = 1000.0 * sum(times) / len(times)
     value = args.batch / (ms / 1000.0)
     what = ("the unmodified reference (StackGAN_v2/model.py + trainer.py train_Dnet / train_Gnet)" if kind == "reference"
-            else "oracle port of the reference (no reference tree on this box)")
+            else "oracle port of the reference (no reference checkout: set SG2_REF)")
     sample = (f"{steps} steps (+{warmup} warm-up) of the {args.branches}-stage train step at batch {args.batch}, {what}, "
               f"fp32 PyTorch CPU, {cores} threads")
     print(json.dumps({
@@ -193,6 +198,35 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ our arm
+DUMP_CAP = 1 << 20        # elements per dumped array: at most 10 arrays x 4 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor, flattened, as out_dir/<name>.npy (float32; float64 stays float64). A tensor of more than DUMP_CAP
+    elements is replaced by DUMP_CAP of its elements at positions fixed by its size (the same on every run and build)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().reshape(-1)
+        if t.numel() > DUMP_CAP:
+            idx = np.sort(np.random.default_rng([1234, t.numel()]).choice(t.numel(), DUMP_CAP, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
+def step_outputs(tr, netG, netsD):
+    """What one train step hands back to its caller: the loss vector [errD_0.., errG_total, kl, cal] and the networks it
+    updated (parameters in the reference's order and OIHW shapes, the EMA copy of G's, floating-point buffers)."""
+    flat = lambda ts: torch.cat([t.detach().reshape(-1).float() for t in ts])
+    out = {"losses": tr.losses, "G_params": flat(netG.parameters()), "G_ema_params": flat(tr.bG.ema_params()),
+           "G_buffers": flat(b for b in netG.buffers() if b.is_floating_point())}
+    for i, d in enumerate(netsD):
+        out[f"D{i}_params"] = flat(d.parameters())
+        out[f"D{i}_buffers"] = flat(b for b in d.buffers() if b.is_floating_point())
+    return out
+
+
 def _shutdown(world, sdist):
     """Leave cleanly. destroy_process_group() used to block forever while CUDA graphs holding captured NCCL collectives
     were alive: the graphs are released first (callers delete them), the group is destroyed on a watchdog, and only if
@@ -401,6 +435,9 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     ms_step = ms_total / steps
     value = world * B / (ms_step / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"images{i}": im for i, im in enumerate(out_imgs)} if synth
+                     else step_outputs(tr, netG, netsD))
 
     step_e2e(0)
     torch.cuda.synchronize()

@@ -1,7 +1,7 @@
 """ORACLE support — generate tests/golden/ref_step_tiny.npz by running the UNMODIFIED reference
 (condGANTrainer.prepare_data / train_Dnet / train_Gnet + EMA, reference G_NET / D_NET*) on CPU in fp32.
 
-    python oracle/make_golden.py            # needs /root/reference (build container only)
+    SG2_REF=<checkout>/StackGAN_v2 python oracle/make_golden.py     # needs a checkout of the reference
 
 The fixture pins oracle/stackgan_oracle.py (tests/test_oracle.py): identical weights + inputs must give the
 reference's losses, logits, images, gradients, BN running statistics and 4-step loss curve.
@@ -15,7 +15,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from oracle import ref_loader  # noqa: E402
+from oracle import golden, ref_loader  # noqa: E402
 from oracle.stackgan_oracle import Cfg, synthetic_batch  # noqa: E402
 
 TINY = dict(GF_DIM=4, DF_DIM=2, EMBEDDING_DIM=8, Z_DIM=10, R_NUM=2, TEXT_DIM=24, BRANCH_NUM=3)
@@ -61,7 +61,7 @@ def run_reference(cfg, batch_size, steps):
 
 def main():
     if not ref_loader.reference_available():
-        raise SystemExit("reference not mounted; golden vectors can only be regenerated in the build container")
+        raise SystemExit("no reference checkout found (set SG2_REF to its StackGAN_v2 directory)")
     cfg = Cfg(**TINY)
     init, rec = run_reference(cfg, BATCH, STEPS)
     out = {"meta_cfg": np.array([TINY[k] for k in sorted(TINY)], dtype=np.int64),
@@ -92,6 +92,7 @@ def main():
         for k, v in sd.items():
             out[f"d{i}_N/" + k] = v.numpy() if "running" in k or "num_batches" in k else np.array(v.double().norm().item())
     out["avg_g_norms"] = np.array([a.double().norm().item() for a in rec["avg_g"]])
+    out = golden.shrink(out)
     path = os.path.join(ROOT, "tests", "golden", "ref_step_tiny.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path), "bytes;", "errD", out["curve_errD"][0], "errG", out["curve_errG"][0])

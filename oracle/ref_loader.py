@@ -1,20 +1,19 @@
-"""ORACLE support — import the UNMODIFIED reference (StackGAN_v2/model.py, trainer.py) in the build container.
+"""ORACLE support — import the UNMODIFIED reference (StackGAN_v2/model.py, trainer.py) from a checkout of it.
 
 Test infrastructure only. The reference needs `easydict` and `tensorboardX` (absent here): two in-memory shims
 are installed before import (SURVEY.md section 8c). cfg is set by assignment (config.py:109 `yaml.load(f)`
 raises under PyYAML 6). Nothing is copied from the reference; it is executed where it lies.
 
-The GPU box has no /root/reference: callers must check `reference_available()`.
+The repository does not ship the reference: callers must check `reference_available()`.
 """
 import os
 import sys
 import types
 
 _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-# $SG2_REF, a driver-provided install under baseline/_ref (git-ignored; never created by this repo: the reference is a
-# Python source tree that must not be copied), or the read-only mount of the build container
-REF_CANDIDATES = [os.environ.get("SG2_REF", ""), os.path.join(_ROOT, "baseline", "_ref", "StackGAN_v2"),
-                  "/root/reference/StackGAN_v2"]
+# $SG2_REF, or a checkout placed under baseline/_ref (git-ignored; never created by this repo: the reference is a
+# Python source tree that must not be copied)
+REF_CANDIDATES = [os.environ.get("SG2_REF", ""), os.path.join(_ROOT, "baseline", "_ref", "StackGAN_v2")]
 
 
 def reference_dir():

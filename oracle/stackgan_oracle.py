@@ -1,13 +1,13 @@
 """ORACLE — test infrastructure only (never imported by the product path).
 
 A plain-PyTorch fp32 restatement of the reference's speech-conditioned StackGAN-v2 train step
-(/root/reference/StackGAN_v2/model.py + trainer.py), written functionally over state dicts that use the
+(StackGAN_v2/model.py + trainer.py), written functionally over state dicts that use the
 reference's own parameter names, so that reference checkpoints load unchanged.
 
 Pinning: the reference ships no tests or golden vectors (SURVEY.md section 4), so this restatement is pinned
-against the reference itself, imported in the build container by oracle/make_golden.py; the outputs are
-committed as tests/golden/*.npz and checked by tests/test_oracle.py (and, where /root/reference is mounted,
-compared directly tensor-by-tensor).
+against the reference itself, imported from a checkout of it by oracle/make_golden.py; the outputs are
+committed as tests/golden/*.npz and checked by tests/test_oracle.py (and, where a reference checkout is given
+with SG2_REF, compared directly tensor-by-tensor).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this file.
 """

@@ -115,3 +115,20 @@ def test_split_k_factor_fills_whole_waves():
                     if s > 1:   # a split launch is a whole number of (nearly) full waves, or a single partial one
                         waves = -(-tiles * s // n_sm)
                         assert tiles * s > (waves - 1) * n_sm + n_sm // 2 or waves == 1, (rows, n, kb, groups, s)
+
+
+def test_bench_dump_outputs_fixed_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: flattened float32 / float64 arrays; a large one is reduced to a sample at positions that
+    depend on its size only, so that two runs (or two builds) can be compared element for element."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_CAP", 100)
+    x = torch.randn(7, 50)
+    arrays = {"big": x, "small": torch.arange(6, dtype=torch.float64), "half": torch.ones(4, dtype=torch.bfloat16)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    a = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in arrays}
+    assert a["big"].dtype == np.float32 and a["big"].shape == (100,) and len(np.unique(a["big"])) == 100
+    assert np.isin(a["big"], x.numpy()).all()
+    assert a["small"].dtype == np.float64 and np.array_equal(a["small"], np.arange(6))
+    assert a["half"].dtype == np.float32 and np.array_equal(a["half"], np.ones(4, np.float32))
+    assert all(np.array_equal(a[n], np.load(tmp_path / "b" / f"{n}.npy")) for n in arrays)

@@ -1,5 +1,6 @@
 """Pin the oracle (oracle/stackgan_oracle.py) to the reference: committed golden vectors produced by the
-unmodified reference (oracle/make_golden.py), and — where /root/reference is mounted — the reference itself."""
+unmodified reference (oracle/make_golden.py), and — where a reference checkout is given (SG2_REF) — the reference
+itself."""
 import os
 
 import numpy as np
@@ -7,6 +8,7 @@ import pytest
 import torch
 
 from oracle import ref_loader
+from oracle.golden import sketch
 from oracle.stackgan_oracle import Cfg, OracleTrainer, param_keys, synthetic_batch
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "ref_step_tiny.npz")
@@ -25,6 +27,14 @@ def _load():
 def _rel(a, b):
     a, b = torch.as_tensor(a).double(), torch.as_tensor(b).double()
     return float((a - b).norm() / (b.norm() + 1e-30))
+
+
+def _rel_ref(z, a, key):
+    """_rel against the reference array `key`, or, for the large ones the fixture keeps as a sketch, the same estimate
+    from the sketches (oracle/golden.py)."""
+    if key in z.files:
+        return _rel(a, z[key])
+    return _rel(sketch(a), z["sketch/" + key])
 
 
 @pytest.fixture(scope="module")
@@ -60,7 +70,7 @@ def test_state_dict_contract(run):
 def test_forward_matches_reference(run):
     z, cfg, tr, outs = run
     o = outs[0]
-    assert _rel(o["fake"][0], z["s0/fake0_full"]) < 1e-5
+    assert _rel_ref(z, o["fake"][0], "s0/fake0_full") < 1e-5
     for i in range(cfg.BRANCH_NUM):
         pooled = torch.nn.functional.adaptive_avg_pool2d(o["fake"][i], 16)
         assert _rel(pooled, z[f"s0/fake{i}_pool16"]) < 1e-5
@@ -84,10 +94,10 @@ def test_gradients_match_reference(run):
     o = outs[0]
     worst = 0.0
     for k, g in o["grads_g"].items():
-        worst = max(worst, _rel(g, z["s0/grad_g/" + k]))
+        worst = max(worst, _rel_ref(z, g, "s0/grad_g/" + k))
     for i, gd in enumerate(o["grads_d"]):
         for k, g in gd.items():
-            worst = max(worst, _rel(g, z[f"s0/grad_d{i}/" + k]))
+            worst = max(worst, _rel_ref(z, g, f"s0/grad_d{i}/" + k))
     assert worst < 2e-4, worst
 
 
@@ -107,9 +117,41 @@ def test_end_state_matches_reference(run):
     np.testing.assert_allclose(norms, z["avg_g_norms"], rtol=1e-4, atol=1e-8)
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference checkout not mounted on this machine")
 def test_direct_against_reference_modules():
-    """Same weights + inputs through the reference's own G_NET / D_NET256 and through the oracle."""
+    """The oracle's module forwards alone (g_forward, d_forward; no trainer, no optimiser) on the reference's initial
+    weights and step-0 batch, against what the reference's own G_NET and D_NET256 produced there: the three images, mu
+    and logvar, and D_NET256's train_Dnet loss (trainer.py:375-427) with the gradient of every D_NET256 weight, which
+    depend on each of its logits and, through backward, on every activation including x_immediate."""
+    from oracle.stackgan_oracle import bce, d_forward, g_forward
+    z, cfg, batch, _, eps_seed, g0, ds = _load()
+    b = synthetic_batch(cfg, batch, seed=1234)
+    torch.manual_seed(eps_seed)
+    eps = torch.FloatTensor(batch, cfg.EMBEDDING_DIM).normal_()          # the draw model.py:190-193 makes
+    fake, mu, logvar = g_forward({k: v.clone() for k, v in g0.items()}, b["z"], b["emb"], eps, cfg, True)
+    assert _rel_ref(z, fake[0], "s0/fake0_full") < 1e-5
+    for i, f in enumerate(fake):
+        assert _rel(torch.nn.functional.adaptive_avg_pool2d(f, 16), z[f"s0/fake{i}_pool16"]) < 1e-5
+    assert _rel(mu, z["s0/mu"]) < 1e-6 and _rel(logvar, z["s0/logvar"]) < 1e-6
+    which = cfg.BRANCH_NUM - 1                                            # D_NET256
+    dsd = {k: v.clone() for k, v in ds[which].items()}
+    keys = param_keys(dsd)
+    for k in keys:
+        dsd[k].requires_grad_(True)
+    ones, zeros, u = torch.ones(batch), torch.zeros(batch), cfg.UNCOND_LOSS
+    rl, _ = d_forward(dsd, b["real"][which], mu, which, cfg)
+    wl, _ = d_forward(dsd, b["wrong"][which], mu, which, cfg)
+    fl, _ = d_forward(dsd, fake[which].detach(), mu, which, cfg)
+    err = (bce(rl[0], ones) + u * bce(rl[1], ones) + bce(wl[0], zeros) + u * bce(wl[1], ones)
+           + bce(fl[0], zeros) + u * bce(fl[1], zeros))
+    np.testing.assert_allclose(float(err.detach()), z["curve_errD"][0][which], rtol=2e-4)
+    grads = torch.autograd.grad(err, [dsd[k] for k in keys])
+    worst = max(_rel_ref(z, g, f"s0/grad_d{which}/" + k) for k, g in zip(keys, grads))
+    assert worst < 2e-4, worst
+
+
+@pytest.mark.skipif(not ref_loader.reference_available(), reason="needs a reference checkout (SG2_REF)")
+def test_direct_against_live_reference_modules():
+    """Same weights + inputs through the reference's own G_NET / D_NET256 (from a checkout) and through the oracle."""
     from oracle.stackgan_oracle import d_forward, g_forward
     cfg = Cfg(GF_DIM=8, DF_DIM=4, EMBEDDING_DIM=16, Z_DIM=12, R_NUM=2, TEXT_DIM=20, BRANCH_NUM=3)
     ref_model, ref_trainer, _ = ref_loader.load_reference(cfg)
