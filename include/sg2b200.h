@@ -104,6 +104,33 @@ int sg2_reduce_slabs(const float* parts, int nslabs, long long n, long long slab
 int sg2_splitk_finish(const float* parts, int nsplit, long long slab, void* y, long long P, int C, int groups,
                       double* stats, const void* epi_src, int epi_mode, void* stream);
 
+/* ---- Inception-v3 scorer (model.py:17-109: torchvision Inception3 in eval mode, run at trainer.py:563-565) ---------
+ * Every BasicConv2d (conv without bias, BatchNorm2d(eps=0.001) on running statistics, ReLU) is one convolution with a
+ * folded bias and ReLU in the epilogue. NHWC bf16 activations; an Inception block's branches write straight into their
+ * channel slice of the block output (no concat).
+ * sg2_conv2d_fprop: y = relu?(conv(x, w) + bias) on the tcgen05 gather kernel; kh x kw <= 32 taps, stride 1 or 2, zero
+ *   padding ph / pw on both sides of each axis (0 = a "valid" convolution). x: the Cin channels of an NHWC tensor whose
+ *   pixel stride is x_ctot channels (a channel slice: pass the slice's first element); y: [B][Ho][Wo] pixels of y_ctot
+ *   channels, Cout of them written. wpk: bf16 [Cout][kh][kw][Cin]; bias: fp32 [Cout] (may be NULL). Cin % 16 == 0,
+ *   Cout, x_ctot, y_ctot % 8 == 0.
+ * sg2_conv2d_plan: the tiling the same call would use, computed from shapes: out[8] = {issued MMA rows, useful rows
+ *   (output pixels), issued MMA columns, BN, BK, tile width, tile height, images per tile}. */
+int sg2_conv2d_fprop(const void* x, int x_ctot, const void* wpk, const float* bias, void* y, int y_ctot, int B, int H,
+                     int W, int Cin, int Cout, int kh, int kw, int stride, int ph, int pw, int relu, void* stream);
+int sg2_conv2d_plan(int B, int H, int W, int Cin, int Cout, int kh, int kw, int stride, int ph, int pw, long long* out);
+/* sg2_inception_stem: img NCHW fp32 [B][3][S][S] in [-1, 1] -> col [B][149][149][32] bf16, the im2col rows of
+ *   Conv2d_1a_3x3 (3x3 s2 p0, K = 27 = (ky, kx, c), zero padded to 32) of the preprocessed image: x * 0.5 + 0.5, per-channel
+ *   (x - mean) / std with the ImageNet mean / std, bilinear resize to 299 x 299 (align_corners=False). No 299^2 image. */
+int sg2_inception_stem(const float* img, void* col, int B, int S, void* stream);
+/* max-pool 3x3 s2 p0 (y may be a channel slice: y_ctot channels per pixel); avg-pool 3x3 s1 p1 count_include_pad=True;
+ * C % 8 == 0. */
+int sg2_maxpool3s2(const void* x, void* y, int y_ctot, int B, int H, int W, int C, void* stream);
+int sg2_avgpool3s1(const void* x, void* y, int B, int H, int W, int C, void* stream);
+/* out [B][C] fp32 = mean over the HW pixels of x [B][HW][C] bf16 (pool3: adaptive 8x8 average, summed in pixel order) */
+int sg2_global_avg(const void* x, float* out, int B, int HW, int C, void* stream);
+/* row softmax, fp32 [M][N] -> [M][N] */
+int sg2_softmax_rows(const float* x, float* y, int M, int N, void* stream);
+
 /* ---- jointConv with the broadcast c_code folded away (NEXT_STAGE_G, model.py:274-279) ---------------------------
  * conv3x3(cat(c (x) 1, h)) = conv3x3_h(h) + bias9[b][border class][o]: the c_code channels are constant over the image,
  * so their share is a per-sample bias that depends only on which taps fall inside the image (sg2_conv_fprop's bias9).

@@ -13,7 +13,7 @@ import sys
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libsg2b200.so")
-SOURCES = ["conv.cu", "elementwise.cu", "small_ops.cu", "precise.cu"]
+SOURCES = ["conv.cu", "elementwise.cu", "small_ops.cu", "precise.cu", "inception.cu"]
 PROBE_SOURCES = ["probe.cu"]          # hardware probes / debug readers: never linked into the product library
 PROBE_LIB_PATH = os.path.join(PKG_DIR, "..", "tools", "libsg2b200_probes.so")
 NVCC_FLAGS = [

@@ -140,7 +140,7 @@ static int pick_tile(int Wg, int Hg, int npix, int* tw, int* th, int* nb) {
 struct GatherDesc {
   View a[4];
   int nmaps;
-  TapF taps[4][16];
+  TapF taps[4][kMaxTaps];
   int ntaps, ngroups;
   int Cin;  // channels per tap (K per tap)
   const void* w;
@@ -156,6 +156,8 @@ struct GatherDesc {
   const float* bias9;  // [B][9][N] border-region bias (tile kernel only)
   const void* epi_src;  // epilogue operand, layout of the output (tile kernel only)
   int epi_mode;         // 0 none, SG2_EPI_ADD, SG2_EPI_LRELU_MASK
+  const float* bias;    // [N] per-channel bias (plain gather kernel only)
+  int tw, th, nb;       // pixel tile of the plain gather kernel (0: pick_tile's 128-pixel tile)
 };
 
 // two pixel tiles per CTA on the gather kernels' 256-channel instances (FpropCfg). Off by default: measured 8.05 vs 7.70
@@ -174,7 +176,11 @@ static int launch_fprop_t(const GatherDesc& d, cudaStream_t st) {
   FpropParams p;
   memset(&p, 0, sizeof(p));
   int rc;
-  if ((rc = pick_tile(d.Wg, d.Hg, kBlockM, &p.tw, &p.th, &p.nb))) return rc;
+  if (d.tw) {
+    p.tw = d.tw, p.th = d.th, p.nb = d.nb;
+  } else if ((rc = pick_tile(d.Wg, d.Hg, kBlockM, &p.tw, &p.th, &p.nb))) {
+    return rc;
+  }
   for (int i = 0; i < d.nmaps; ++i)
     if ((rc = make_act_map(&p.tmA[i], d.a[i], BK, p.tw, p.th, p.nb))) return rc;
   const long long K = (long long)d.ntaps * d.Cin;
@@ -183,6 +189,7 @@ static int launch_fprop_t(const GatherDesc& d, cudaStream_t st) {
   p.ntaps = d.ntaps;
   p.kchunks = d.Cin / BK;
   p.ngroups = d.ngroups;
+  p.bias = d.bias;
   const int KB = p.ntaps * p.kchunks;
   p.splitk = d.splitk < 1 ? 1 : (d.splitk > KB ? KB : d.splitk);
   if (p.splitk > 1 && d.out_mode == OUT_BF16) SG2_FAIL(SG2_EINVAL, "split-K needs an fp32 output mode");
@@ -221,7 +228,7 @@ static int launch_fprop_t(const GatherDesc& d, cudaStream_t st) {
     if (e != cudaSuccess) SG2_FAIL((int)e, "cudaFuncSetAttribute(fprop<%d,%d>): %s", BN, BK, cudaGetErrorString(e));
   }
   const int pix_tiles = p.tiles_x * p.tiles_y * p.tiles_b;
-  dim3 grid((pix_tiles + MT - 1) / MT, d.N / BN, p.ngroups * p.splitk);
+  dim3 grid((pix_tiles + MT - 1) / MT, (d.N + BN - 1) / BN, p.ngroups * p.splitk);
   igemm_fprop_kernel<BN, BK, MT><<<grid, kNumThreads, smem, st>>>(p);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) SG2_FAIL((int)e, "fprop<%d,%d> launch: %s", BN, BK, cudaGetErrorString(e));
@@ -639,6 +646,19 @@ static int gather_tiles(const GatherDesc& d) {
   return ((d.Wg + tw - 1) / tw) * ((d.Hg + th - 1) / th) * ((d.B + nb - 1) / nb);
 }
 
+// the plain gather kernel (one 128 x bn tile per CTA)
+static int launch_fprop_plain(const GatherDesc& d, int bn, int bk, cudaStream_t st) {
+#define SG2_CASE(BN_, BK_) \
+  if (bn == BN_ && bk == BK_) return launch_fprop_t<BN_, BK_>(d, st);
+  SG2_CASE(256, 64) SG2_CASE(128, 64) SG2_CASE(64, 64) SG2_CASE(32, 64)
+  SG2_CASE(256, 32) SG2_CASE(128, 32) SG2_CASE(64, 32) SG2_CASE(32, 32)
+  SG2_CASE(256, 16) SG2_CASE(128, 16) SG2_CASE(64, 16) SG2_CASE(32, 16)
+  SG2_CASE(16, 64) SG2_CASE(16, 32) SG2_CASE(16, 16)
+  SG2_CASE(160, 64) SG2_CASE(160, 32) SG2_CASE(192, 64) SG2_CASE(192, 32)
+#undef SG2_CASE
+  SG2_FAIL(SG2_EINVAL, "no fprop instance for BN=%d BK=%d", bn, bk);
+}
+
 static int launch_fprop(const GatherDesc& d, cudaStream_t st) {
   if (d.Cin % 16) SG2_FAIL(SG2_EINVAL, "K per tap (%d) must be a multiple of 16", d.Cin);
   if (d.N % 16) SG2_FAIL(SG2_EINVAL, "N (%d) must be a multiple of 16", d.N);
@@ -669,15 +689,7 @@ static int launch_fprop(const GatherDesc& d, cudaStream_t st) {
   }
   if (d.epi_mode) SG2_FAIL(SG2_ENOFUSE, "epilogue operand: this shape runs on the gather kernel (K %d, N %d)", d.Cin, d.N);
   if (bn == 256 && bk == 64 && igemm_mt2() && gather_tiles(d) >= 2) return launch_fprop_t<256, 64, 2>(d, st);
-#define SG2_CASE(BN_, BK_) \
-  if (bn == BN_ && bk == BK_) return launch_fprop_t<BN_, BK_>(d, st);
-  SG2_CASE(256, 64) SG2_CASE(128, 64) SG2_CASE(64, 64) SG2_CASE(32, 64)
-  SG2_CASE(256, 32) SG2_CASE(128, 32) SG2_CASE(64, 32) SG2_CASE(32, 32)
-  SG2_CASE(256, 16) SG2_CASE(128, 16) SG2_CASE(64, 16) SG2_CASE(32, 16)
-  SG2_CASE(16, 64) SG2_CASE(16, 32) SG2_CASE(16, 16)
-  SG2_CASE(160, 64) SG2_CASE(160, 32) SG2_CASE(192, 64) SG2_CASE(192, 32)
-#undef SG2_CASE
-  SG2_FAIL(SG2_EINVAL, "no fprop instance for BN=%d BK=%d", bn, bk);
+  return launch_fprop_plain(d, bn, bk, st);
 }
 
 static inline int fdiv2(int v) { return v >= 0 ? v / 2 : -((-v + 1) / 2); }  // floor(v/2)
@@ -977,11 +989,146 @@ static int launch_wgrad(const WgradDesc& d, cudaStream_t st) {
 static const int kS2_kh[2][2] = {{1, 3}, {2, 0}};   // [parity][a]
 static const int kS2_dy[2][2] = {{0, -1}, {0, 1}};  // [parity][a] : output row = i + dy
 
+// ------------------------------------------------------------------------------------------ general convolution
+// sg2_conv2d_fprop: kh x kw, stride 1 or 2, zero padding, bias + ReLU, channel slices in and out, on the plain gather
+// kernel. The pixel tile is the rectangle of at most 128 output pixels that covers the map in the fewest tiles: a partial
+// TMA box fills tw*th*nb rows of the 128-row operand, the rest of the MMA rows are issued but never stored. A stride-1
+// 1x1 convolution walks the pixels of the whole batch as one row (no waste but the last tile's tail).
+struct Conv2dGeo {
+  int Ho, Wo, flat, tw, th, nb, bn, bk;
+  long long tiles;
+};
+
+// output tile width: the smallest gather instance that covers N (weight rows past N are TMA zero fill), else the
+// instance with the least padded width
+static int conv2d_bn(int N, int bk) {
+  static const int wide[] = {16, 32, 64, 128, 160, 192, 256};
+  static const int narrow[] = {16, 32, 64, 128, 256};   // BK = 16 has no 160 / 192 instances
+  const int* c = bk == 16 ? narrow : wide;
+  const int nc = bk == 16 ? 5 : 7;
+  for (int i = 0; i < nc; ++i)
+    if (c[i] >= N) return c[i];
+  int best = 256;
+  for (int i = nc - 1; i >= 0 && c[i] >= 128; --i)
+    if ((long long)((N + c[i] - 1) / c[i]) * c[i] < (long long)((N + best - 1) / best) * best) best = c[i];
+  return best;
+}
+
+static int conv2d_geo(int B, int H, int W, int Cin, int Cout, int kh, int kw, int stride, int ph, int pw, Conv2dGeo& g) {
+  if (B < 1 || H < 1 || W < 1) SG2_FAIL(SG2_EINVAL, "conv2d: empty input %dx%dx%d", B, H, W);
+  if (Cin < 16 || Cin % 16) SG2_FAIL(SG2_EINVAL, "conv2d: Cin %d must be a multiple of 16", Cin);
+  if (Cout < 8 || Cout % 8) SG2_FAIL(SG2_EINVAL, "conv2d: Cout %d must be a multiple of 8", Cout);
+  if (stride != 1 && stride != 2) SG2_FAIL(SG2_EINVAL, "conv2d: stride %d (1 or 2)", stride);
+  if (kh < 1 || kw < 1 || kh * kw > kMaxTaps) SG2_FAIL(SG2_EINVAL, "conv2d: %dx%d kernel (at most %d taps)", kh, kw, kMaxTaps);
+  if (ph < 0 || pw < 0 || ph >= kh || pw >= kw) SG2_FAIL(SG2_EINVAL, "conv2d: padding (%d, %d) for a %dx%d kernel", ph, pw, kh, kw);
+  if (stride == 2 && (H < 2 || W < 2)) SG2_FAIL(SG2_EINVAL, "conv2d: stride 2 on a %dx%d map", H, W);
+  g.Ho = (H + 2 * ph - kh) / stride + 1;
+  g.Wo = (W + 2 * pw - kw) / stride + 1;
+  if (H + 2 * ph < kh || W + 2 * pw < kw) SG2_FAIL(SG2_EINVAL, "conv2d: %dx%d kernel larger than the padded map", kh, kw);
+  g.bk = (Cin % 64 == 0) ? 64 : ((Cin % 32 == 0) ? 32 : 16);
+  g.bn = conv2d_bn(Cout, g.bk);
+  g.flat = kh == 1 && kw == 1 && stride == 1;
+  if (g.flat) {
+    const long long P = (long long)B * H * W;
+    if (P > 0x7fffffffLL) SG2_FAIL(SG2_EINVAL, "conv2d: %lld pixels", P);
+    g.tw = P < kBlockM ? (int)P : kBlockM, g.th = 1, g.nb = 1;
+    g.tiles = (P + g.tw - 1) / g.tw;
+    return 0;
+  }
+  if (g.Ho * g.Wo <= kBlockM) {
+    g.tw = g.Wo, g.th = g.Ho;
+    g.nb = kBlockM / (g.Ho * g.Wo);
+    if (g.nb > B) g.nb = B;
+  } else {
+    long long best = -1;
+    for (int tw = 1; tw <= (g.Wo < kBlockM ? g.Wo : kBlockM); ++tw) {
+      int th = kBlockM / tw;
+      if (th > g.Ho) th = g.Ho;
+      const long long t = (long long)((g.Wo + tw - 1) / tw) * ((g.Ho + th - 1) / th);
+      if (best < 0 || t <= best) best = t, g.tw = tw, g.th = th;   // ties: the wider tile
+    }
+    g.nb = 1;
+  }
+  g.tiles = (long long)((g.Wo + g.tw - 1) / g.tw) * ((g.Ho + g.th - 1) / g.th) * ((B + g.nb - 1) / g.nb);
+  return 0;
+}
+
 }  // namespace sg2
 
 using namespace sg2;
 
 extern "C" {
+
+int sg2_conv2d_plan(int B, int H, int W, int Cin, int Cout, int kh, int kw, int stride, int ph, int pw,
+                    long long* out) {
+  Conv2dGeo g;
+  const int rc = conv2d_geo(B, H, W, Cin, Cout, kh, kw, stride, ph, pw, g);
+  if (rc) return rc;
+  const long long v[8] = {g.tiles * kBlockM, (long long)B * g.Ho * g.Wo, (long long)((Cout + g.bn - 1) / g.bn) * g.bn,
+                          g.bn, g.bk, g.tw, g.th, g.nb};
+  memcpy(out, v, sizeof(v));
+  return 0;
+}
+
+int sg2_conv2d_fprop(const void* x, int x_ctot, const void* wpk, const float* bias, void* y, int y_ctot, int B, int H,
+                     int W, int Cin, int Cout, int kh, int kw, int stride, int ph, int pw, int relu, void* stream) {
+  Conv2dGeo g;
+  int rc = conv2d_geo(B, H, W, Cin, Cout, kh, kw, stride, ph, pw, g);
+  if (rc) return rc;
+  if (x_ctot < Cin || (x_ctot % 8) || y_ctot < Cout || (y_ctot % 8))
+    SG2_FAIL(SG2_EINVAL, "conv2d: channel strides %d / %d (multiples of 8, >= Cin %d / Cout %d)", x_ctot, y_ctot, Cin, Cout);
+  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(wpk)) & 15)
+    SG2_FAIL(SG2_EINVAL, "conv2d: operands must be 16-byte aligned");
+  if (relu != 0 && relu != 1) SG2_FAIL(SG2_EINVAL, "conv2d: relu %d", relu);
+  GatherDesc d;
+  memset(&d, 0, sizeof(d));
+  d.Cin = Cin;
+  d.w = wpk;
+  d.N = Cout;
+  d.out = y;
+  d.out_mode = OUT_BF16;
+  d.splitk = 1;
+  d.bias = bias;
+  d.act = relu ? 3 : 0;
+  d.ngroups = 1;
+  d.tw = g.tw, d.th = g.th, d.nb = g.nb;
+  const __nv_bfloat16* xb = reinterpret_cast<const __nv_bfloat16*>(x);
+  if (g.flat) {
+    const int P = B * H * W;
+    d.a[0] = View{xb, Cin, P, 1, 1, (long long)x_ctot, (long long)P * x_ctot, (long long)P * x_ctot};
+    d.nmaps = 1;
+    d.ntaps = 1;
+    d.taps[0][0] = TapF{0, 0, 0, 0};
+    d.Wg = P, d.Hg = 1, d.B = 1;
+    d.osx = y_ctot, d.osy = (long long)P * y_ctot, d.osb = d.osy;
+  } else {
+    const View xv{xb, Cin, W, H, B, (long long)x_ctot, (long long)W * x_ctot, (long long)H * W * x_ctot};
+    if (stride == 1) {
+      d.a[0] = xv;
+      d.nmaps = 1;
+    } else {   // parity plane (py, px): input pixels (2i + py, 2j + px)
+      for (int py = 0; py < 2; ++py)
+        for (int px = 0; px < 2; ++px) {
+          View v = xv;
+          v.base = xv.base + py * xv.sy + px * xv.sx;
+          v.H = (H - py + 1) / 2, v.W = (W - px + 1) / 2;
+          v.sy = 2 * xv.sy, v.sx = 2 * xv.sx;
+          d.a[py * 2 + px] = v;
+        }
+      d.nmaps = 4;
+    }
+    d.ntaps = kh * kw;
+    for (int ky = 0; ky < kh; ++ky)
+      for (int kx = 0; kx < kw; ++kx) {
+        const int ry = ky - ph, rx = kx - pw;   // input row = stride * oy + ry
+        d.taps[0][ky * kw + kx] = stride == 1 ? TapF{0, (int8_t)ry, (int8_t)rx, 0}
+                                              : TapF{(int8_t)((ry & 1) * 2 + (rx & 1)), (int8_t)fdiv2(ry), (int8_t)fdiv2(rx), 0};
+      }
+    d.Wg = g.Wo, d.Hg = g.Ho, d.B = B;
+    d.osx = y_ctot, d.osy = (long long)g.Wo * y_ctot, d.osb = (long long)g.Ho * g.Wo * y_ctot;
+  }
+  return launch_fprop_plain(d, g.bn, g.bk, (cudaStream_t)stream);
+}
 
 int sg2_version(void) { return 2; }
 int sg2_set_sm_reserve(int n_sms) {

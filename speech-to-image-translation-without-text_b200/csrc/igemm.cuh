@@ -22,13 +22,14 @@ constexpr int kNumThreads = 192;  // warp0: TMA producer, warp1: MMA issuer + TM
 struct TapF {
   int8_t map, dy, dx, pad;
 };
+constexpr int kMaxTaps = 32;   // per group: up to 5x5 (sg2_conv2d_fprop)
 
 enum OutMode : int { OUT_BF16 = 0, OUT_F32_ATOMIC = 1, OUT_F32_STORE = 2 };
 
 struct FpropParams {
   CUtensorMap tmA[4];
   CUtensorMap tmB;
-  TapF taps[4][16];  // [group][tap]
+  TapF taps[4][kMaxTaps];  // [group][tap]
   int ntaps, kchunks;
   int ngroups, splitk;
   int tw, th, nb;
@@ -42,7 +43,8 @@ struct FpropParams {
   int stages;
   double* stats;  // optional [groups][2][N] fp64: per-channel sum / sum of squares of the (bf16-rounded) outputs, += (BN statistics)
   int stats_bg;  // images per statistics group (0: one group); a tile never straddles groups (checked on the host)
-  int act;       // epilogue activation: 0 none, 2 LeakyReLU(0.2) (layers without BatchNorm: the D stems)
+  int act;       // epilogue activation: 0 none, 2 LeakyReLU(0.2) (layers without BatchNorm: the D stems), 3 ReLU
+  const float* bias;  // optional [N] fp32, added before the activation (igemm_fprop_kernel only)
   // cluster split-K (igemm_fprop_cluster_kernel): bf16 output, the `splitk` CTAs of a tile form a cluster and reduce
   // their partial tiles through distributed shared memory in rank order
   const void* epi_src;     // optional epilogue operand (layout of the output, bf16), see sg2_conv_dgrad
@@ -125,12 +127,14 @@ __global__ void __launch_bounds__(kNumThreads) igemm_fprop_kernel(const __grid_c
   // descriptors in uniform registers and emits back-to-back UTCHMMA/UTMALDG. A divergent `if (lane == 0)` body costs
   // ~146 cycles per tcgen05.mma (tools/probe_mma.py) against a 64-cycle tensor floor at N = 128.
   if (warp == 0) {
+    // a pixel tile may be a partial box (tw * th * nb < 128 rows, sg2_conv2d_fprop): only its bytes arrive
+    const uint32_t tx_bytes = uint32_t(MT * p.tw * p.th * p.nb * BK * 2 + Cfg::kBBytes);
     int s = 0;
     uint32_t ph = 0;
     for (int it = 0; it < nkb; ++it) {
       mbar_wait(&empty[s], ph ^ 1);
       if (elect_one()) {
-        mbar_expect_tx(&full[s], Cfg::kStageBytes);
+        mbar_expect_tx(&full[s], tx_bytes);
         const int kb = kb_begin + it;
         const int tap = kb / p.kchunks;
         const int ch = kb - tap * p.kchunks;
@@ -187,6 +191,9 @@ __global__ void __launch_bounds__(kNumThreads) igemm_fprop_kernel(const __grid_c
     const int xi = row % p.tw;
     const int yi = (row / p.tw) % p.th;
     const int bi = row / (p.tw * p.th);
+    // the rows past a partial box hold stale shared memory: their accumulators are never stored
+    const bool in_box = row < p.tw * p.th * p.nb;
+    const int ncols = p.N - n0;   // < BN: the weight box ran past N (zero filled); those columns are not stored
     const bool do_stats = (p.stats != nullptr) && (p.out_mode == OUT_BF16);
     const int et = threadIdx.x - 64;  // 0..127 within the epilogue warps
     constexpr int SN = BN < 32 ? 32 : BN;
@@ -197,7 +204,7 @@ __global__ void __launch_bounds__(kNumThreads) igemm_fprop_kernel(const __grid_c
     const bool second = MT == 2 && m == 1;
     const int x0m = second ? x0[MT - 1] : x0[0], y0m = second ? y0[MT - 1] : y0[0], b0m = second ? b0[MT - 1] : b0[0];
     const int x = x0m + xi, y = y0m + yi, b = b0m + bi;
-    const bool valid = (x < p.Wo) && (y < p.Ho) && (b < p.B);
+    const bool valid = in_box && (x < p.Wo) && (y < p.Ho) && (b < p.B);
     const long long off = p.out_off[g] + (long long)b * p.sb + (long long)y * p.sy + (long long)x * p.sx + n0 +
                           (p.out_mode == OUT_F32_STORE ? (long long)split * p.split_stride : 0);
     const uint32_t taddr = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(m * BN);
@@ -210,12 +217,20 @@ __global__ void __launch_bounds__(kNumThreads) igemm_fprop_kernel(const __grid_c
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = 0u;
       }
+      if (p.bias) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (c0 + j < ncols) v[j] = __float_as_uint(__uint_as_float(v[j]) + __ldg(p.bias + n0 + c0 + j));
+      }
       if (p.act == 2) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const float f = __uint_as_float(v[j]);
           v[j] = __float_as_uint(f > 0.f ? f : 0.2f * f);
         }
+      } else if (p.act == 3) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) v[j] = __float_as_uint(fmaxf(__uint_as_float(v[j]), 0.f));
       }
       if (do_stats) {
         // statistics of what BatchNorm will read back: the bf16-rounded outputs of the valid rows
@@ -238,6 +253,7 @@ __global__ void __launch_bounds__(kNumThreads) igemm_fprop_kernel(const __grid_c
           uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.out) + off + c0);
 #pragma unroll
           for (int j = 0; j < (BN < 32 ? BN / 8 : 4); ++j) {
+            if (c0 + 8 * j >= ncols) break;
             uint4 o;
             o.x = pack_bf16x2(__uint_as_float(v[8 * j + 0]), __uint_as_float(v[8 * j + 1]));
             o.y = pack_bf16x2(__uint_as_float(v[8 * j + 2]), __uint_as_float(v[8 * j + 3]));

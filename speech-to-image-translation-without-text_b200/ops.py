@@ -701,3 +701,78 @@ def logits_bwd(dprob, prob, x, w, dx, dx_accumulate, dw, dbias):
         scratch = torch.empty(_lib.lib().sg2_logits_bwd_scratch_floats(B, H * W, C), device=x.device, dtype=torch.float32)
     _call("sg2_logits_bwd", 1 + (dw is not None), _p(dprob), _p(prob), _p(x), _p(w), _p(dx), int(dx_accumulate), _p(dw),
           _p(dbias), _p(scratch), B, H * W, C, _st())
+
+
+# ------------------------------------------------------------------------------------------ Inception-v3 scorer
+def _slice_ptr(t, c0):
+    """Device pointer of channel c0 of the NHWC tensor t (its pixel stride stays t.shape[-1] channels)."""
+    if t.dtype != torch.bfloat16:
+        raise RuntimeError("sg2b200: Inception activations are bf16")
+    return _p(t) + 2 * c0
+
+
+def conv2d_out_hw(H, W, kh, kw, stride, ph, pw):
+    return (H + 2 * ph - kh) // stride + 1, (W + 2 * pw - kw) // stride + 1
+
+
+def conv2d_plan(B, H, W, Cin, Cout, kh, kw, stride=1, ph=0, pw=0):
+    """The tiling sg2_conv2d_fprop uses for this shape: dict of issued / useful MMA rows and columns, BN, BK, tile."""
+    out = (ctypes.c_longlong * 8)()
+    _lib.call("sg2_conv2d_plan", B, H, W, Cin, Cout, kh, kw, stride, ph, pw, ctypes.addressof(out))
+    keys = ("issued_rows", "useful_rows", "issued_cols", "bn", "bk", "tw", "th", "nb")
+    return dict(zip(keys, (int(v) for v in out)))
+
+
+def conv2d_fprop(x, Cin, wpk, bias, out, Cout, kh, kw, stride=1, ph=0, pw=0, relu=True, x_c0=0, out_c0=0):
+    """out[..., out_c0:out_c0+Cout] = relu?(conv(x[..., x_c0:x_c0+Cin], wpk) + bias); x, out NHWC bf16 (B, H, W, C)."""
+    B, H, W, _ = x.shape
+    Ho, Wo = conv2d_out_hw(H, W, kh, kw, stride, ph, pw)
+    if tuple(out.shape[:3]) != (B, Ho, Wo) or x_c0 + Cin > x.shape[3] or out_c0 + Cout > out.shape[3]:
+        raise RuntimeError(f"sg2b200: conv2d_fprop: shapes {tuple(x.shape)} -> {tuple(out.shape)} "
+                           f"({kh}x{kw} s{stride}, channels {x_c0}+{Cin} -> {out_c0}+{Cout})")
+    flops = 2.0 * B * Ho * Wo * Cout * Cin * kh * kw
+    _conv_call("sg2_conv2d_fprop", 1, flops, _slice_ptr(x, x_c0), x.shape[3], _p(wpk), _p(bias),
+               _slice_ptr(out, out_c0), out.shape[3], B, H, W, Cin, Cout, kh, kw, stride, ph, pw, int(relu), _st())
+    return out
+
+
+def inception_stem(img):
+    """(B,3,S,S) fp32 in [-1, 1] -> (B,149,149,32) bf16 im2col rows of Conv2d_1a_3x3 of the preprocessed 299^2 image."""
+    B, _, S, _ = img.shape
+    col = torch.empty((B, 149, 149, 32), device=img.device, dtype=torch.bfloat16)
+    _call("sg2_inception_stem", 1, _p(img), _p(col), B, S, _st())
+    return col
+
+
+def maxpool3s2(x, out=None, out_c0=0):
+    B, H, W, C = x.shape
+    Ho, Wo = (H - 3) // 2 + 1, (W - 3) // 2 + 1
+    if out is None:
+        out = torch.empty((B, Ho, Wo, C), device=x.device, dtype=torch.bfloat16)
+    if tuple(out.shape[:3]) != (B, Ho, Wo) or out_c0 + C > out.shape[3]:
+        raise RuntimeError("sg2b200: maxpool3s2: bad output")
+    _call("sg2_maxpool3s2", 1, _p(x), _slice_ptr(out, out_c0), out.shape[3], B, H, W, C, _st())
+    return out
+
+
+def avgpool3s1(x):
+    B, H, W, C = x.shape
+    out = torch.empty_like(x)
+    _call("sg2_avgpool3s1", 1, _p(x), _p(out), B, H, W, C, _st())
+    return out
+
+
+def global_avg(x, out=None):
+    B, H, W, C = x.shape
+    if out is None:
+        out = torch.empty((B, C), device=x.device, dtype=torch.float32)
+    _call("sg2_global_avg", 1, _p(x), _p(out), B, H * W, C, _st())
+    return out
+
+
+def softmax_rows(x, out=None):
+    M, N = x.shape
+    if out is None:
+        out = torch.empty_like(x)
+    _call("sg2_softmax_rows", 1, _p(x), _p(out), M, N, _st())
+    return out

@@ -307,9 +307,10 @@ class FusedTrainer:
             self._sO = [torch.cuda.Stream(device=self.dev, priority=(prio + [0])[i]) if two else None for i in range(n + 1)]
         return self._sD
 
-    def step(self, z, emb, real, wrong, labels, eps=None):
+    def step(self, z, emb, real, wrong, labels, eps=None, on_img=None):
         """z (B,Z) f32, emb (B,T) f32, real/wrong: lists of (B,3,S,S) f32 NCHW, labels (B,) int32 — all on the GPU.
-        Returns the device tensor [errD_0.., errG_total, kl, cal] (no host sync).
+        Returns the device tensor [errD_0.., errG_total, kl, cal] (no host sync). on_img(i, img): called on the current
+        stream as soon as stage i's fake image has been issued (CapturedStep forks the Inception scoring there).
 
         Scheduling: the G forward runs on the current stream; the three discriminators are independent of one another
         (own weights, own optimiser, own image scale), so each D's update AND its part of the G step (forward on the
@@ -359,12 +360,14 @@ class FusedTrainer:
         def on_mu(mu_):
             hook["mu3"] = mu_.repeat(3, 1) if self.batched_d else None
 
-        def on_img(i_, img_):
+        def on_img_(i_, img_):
             if early and i_ < nD:
                 hook["ev"][i_] = torch.cuda.Event()
                 hook["ev"][i_].record(main)
+            if on_img is not None:
+                on_img(i_, img_)
 
-        fake, mu, logvar, Tg = self.G.forward(z, emb, eps, True, on_mu=on_mu, on_img=on_img)  # trainer.py:544
+        fake, mu, logvar, Tg = self.G.forward(z, emb, eps, True, on_mu=on_mu, on_img=on_img_)  # trainer.py:544
         mu3 = hook["mu3"]
         dmu = torch.empty_like(mu)
         dlogvar = torch.empty_like(logvar)
@@ -470,14 +473,23 @@ class CapturedStep:
     once into a CUDA graph and replayed per step: the launch-bound inner loop costs one cudaGraphLaunch instead of
     ~20 ms of Python/ctypes/driver work. Inputs live in static device buffers (`load()` copies a batch in)."""
 
-    def __init__(self, trainer, batch_size, warmup=3, draw_noise=True):
+    def __init__(self, trainer, batch_size, warmup=3, draw_noise=True, scorer=None, score_real=True):
         """draw_noise: the graph draws z ~ N(0,1) (trainer.py:542) and the reparameterisation eps (model.py:190-193) itself
         (Philox state advanced per replay); False: both come from the static buffers `noise` / `eps` filled by load()
-        (parity tests replay the graph on given noise)."""
+        (parity tests replay the graph on given noise).
+        scorer: an sg2b200.inception.INCEPTION_V3; the graph then also scores this step's last fake image and (score_real)
+        the static real[-1] into `pred_fake` / `pool3_fake` / `pred_real` / `pool3_real`, what trainer.py:563-565
+        computes. The scoring forks off the main stream once the last image is issued, runs on its own stream at normal
+        priority (below the chain streams') and joins before the graph ends; it writes no training state."""
         self.tr = trainer
         cfg, dev = trainer.cfg, trainer.dev
         B = batch_size
         self.draw_noise = draw_noise
+        self.scorer, self.score_real = scorer, score_real
+        if scorer is not None:
+            self._s_score = torch.cuda.Stream(device=dev, priority=0)
+            self.pred_fake, self.pred_real = (torch.zeros(B, 1000, device=dev) for _ in range(2))
+            self.pool3_fake, self.pool3_real = (torch.zeros(B, 2048, device=dev) for _ in range(2))
         self.noise = torch.zeros(B, cfg.GAN.Z_DIM, device=dev)
         self.eps = torch.zeros(B, cfg.GAN.EMBEDDING_DIM, device=dev)
         self.emb = torch.zeros(B, cfg.TEXT.DIMENSION, device=dev)
@@ -501,11 +513,31 @@ class CapturedStep:
             d.copy_(s, non_blocking=non_blocking)
         self.labels.copy_(labels, non_blocking=non_blocking)
 
+    def _score(self, i, img):
+        if i != len(self.tr.Ds) - 1:
+            return
+        fork = torch.cuda.Event()
+        fork.record(torch.cuda.current_stream())
+        s = self._s_score
+        s.wait_event(fork)
+        img.record_stream(s)
+        with torch.cuda.stream(s):                                         # trainer.py:563-565
+            self.scorer(img, out=(self.pred_fake, self.pool3_fake))
+            if self.score_real:
+                self.scorer(self.real[-1], out=(self.pred_real, self.pool3_real))
+        self._scored = torch.cuda.Event()
+        self._scored.record(s)
+
     def _body(self):
+        hook = self._score if self.scorer is not None else None
         if self.draw_noise:
             self.noise.normal_(0, 1)                                       # trainer.py:542
-            return self.tr.step(self.noise, self.emb, self.real, self.wrong, self.labels)
-        return self.tr.step(self.noise, self.emb, self.real, self.wrong, self.labels, eps=self.eps)
+            losses = self.tr.step(self.noise, self.emb, self.real, self.wrong, self.labels, on_img=hook)
+        else:
+            losses = self.tr.step(self.noise, self.emb, self.real, self.wrong, self.labels, eps=self.eps, on_img=hook)
+        if hook is not None:
+            torch.cuda.current_stream().wait_event(self._scored)
+        return losses
 
     def capture(self):
         side = torch.cuda.Stream(device=self.tr.dev)

@@ -83,14 +83,25 @@ def patch_reference_trainer(trainer_module):
     return trainer_module
 
 
-def install_as_reference_model():
+def install_as_reference_model(inception=False):
     """Make `from model import G_NET, D_NET64, ...` (trainer.py:24) resolve to sg2b200.model, so the reference's
     unmodified main.py / trainer.py run on the CUDA kernels: call before importing the reference's trainer.
     Also binds the reference's global cfg (miscc.config.cfg) and arranges for the reference trainer's load_params
-    (writes through `.data`) to invalidate the kernels' operand caches."""
+    (writes through `.data`) to invalidate the kernels' operand caches.
+    inception=True: the aliased module is a proxy of sg2b200.model whose INCEPTION_V3 is the native scorer
+    (sg2b200.inception), so the trainer's in-loop scoring (trainer.py:563-565) runs on these kernels too;
+    sg2b200.model.INCEPTION_V3 itself is unchanged."""
     import sys
+    import types
     from . import config, model
-    sys.modules["model"] = model
+    if inception:
+        from . import inception as inc
+        proxy = types.ModuleType("model", model.__doc__)
+        proxy.__dict__.update({k: v for k, v in vars(model).items() if not k.startswith("__")})
+        proxy.INCEPTION_V3 = inc.INCEPTION_V3
+        sys.modules["model"] = proxy
+    else:
+        sys.modules["model"] = model
     config.bind_reference_cfg()
     if "trainer" in sys.modules:
         patch_reference_trainer(sys.modules["trainer"])
