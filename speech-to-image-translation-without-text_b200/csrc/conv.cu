@@ -977,9 +977,10 @@ static int launch_wgrad(const WgradDesc& d, cudaStream_t st) {
 #define SG2_CASE(BN_, A_, B_) \
   if (bn == BN_ && cwa == A_ && cwb == B_) return launch_wgrad_t<BN_, A_, B_>(d, st);
   SG2_CASE(256, 64, 64) SG2_CASE(128, 64, 64) SG2_CASE(64, 64, 64)
-  SG2_CASE(256, 64, 32) SG2_CASE(128, 64, 32) SG2_CASE(64, 64, 32) SG2_CASE(32, 64, 32)
+  // (BN 64, CWB 32) cannot occur: BN = 64 means 32 < Cin <= 64, and the only multiple of 32 there is 64 (CWB = 64)
+  SG2_CASE(256, 64, 32) SG2_CASE(128, 64, 32) SG2_CASE(32, 64, 32)
   SG2_CASE(256, 32, 64) SG2_CASE(128, 32, 64) SG2_CASE(64, 32, 64)
-  SG2_CASE(256, 32, 32) SG2_CASE(128, 32, 32) SG2_CASE(64, 32, 32) SG2_CASE(32, 32, 32)
+  SG2_CASE(256, 32, 32) SG2_CASE(128, 32, 32) SG2_CASE(32, 32, 32)
   SG2_CASE(16, 64, 16) SG2_CASE(16, 32, 16)
 #undef SG2_CASE
   SG2_FAIL(SG2_EINVAL, "no wgrad instance for BN=%d CWA=%d CWB=%d", bn, cwa, cwb);
